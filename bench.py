@@ -22,6 +22,11 @@ Prints ONE JSON line (rank 0):
              rank 0 to every rank with an NCCL broadcast per step (double-buffered against the previous block's kernel)
   cpu_baseline  the compiled reference (oracle/_ref) or the oracle port on this box's host cores, bounded sample
 --impl reference: the reference's own CPU implementation of the same step on all host threads (rank 0 only).
+
+--dump-outputs DIR (rank 0): after the K timed steps, what the last step handed its caller, for comparing two builds output for output
+(the inputs are seeded, so they are the same in every run):
+  fir_bank_out.npy       float32 (256, 16384, 2): I,Q of every channel at DUMP_COLS fixed output positions (all 239 981 would be 491 MB)
+  fir_bank_out_cols.npy  float64 (16384,): those positions -- the first and last 1024 outputs and a seeded sample in between
 """
 from __future__ import annotations
 
@@ -44,6 +49,21 @@ CHANNELS, N_IN, TAPS, DECIM = 256, 2_400_000, 199, 10
 WORKLOAD = "256-channel fir_decimate_cc bank, decim=10, 199-tap HAMMING, 2.4 Msps/ch synthetic cf32 (BASELINE configs[1])"
 METRIC = "Msamples/s in, 256-ch fir_decimate_cc d=10"
 ALGO_BYTES_PER_SAMPLE = 8.0 + 8.0 / DECIM            # SURVEY 8(d): 8 B read per input sample + 8 B written per output
+DUMP_COLS, DUMP_EDGE = 16384, 1024
+
+
+def dump_columns(n_out: int) -> np.ndarray:
+    """output positions --dump-outputs keeps: both ends of the stream (filter start-up and the last complete window) and a seeded sample between"""
+    mid = np.random.default_rng(0).choice(np.arange(DUMP_EDGE, n_out - DUMP_EDGE), DUMP_COLS - 2 * DUMP_EDGE, replace=False)
+    return np.sort(np.concatenate([np.arange(DUMP_EDGE), mid, np.arange(n_out - DUMP_EDGE, n_out)]))
+
+
+def dump_outputs(out_dir: str, arrays: dict) -> None:
+    d = Path(out_dir)
+    d.mkdir(parents=True, exist_ok=True)
+    for name, a in arrays.items():
+        assert a.dtype in (np.float32, np.float64), (name, a.dtype)
+        np.save(d / f"{name}.npy", a)
 
 
 def base_config(world: int) -> dict:
@@ -301,7 +321,12 @@ def run_b200(args):
         launches0 = csdr_b200.kernel_launches()
         total_ms, per_kernel_ms = timed_loop(fir_step, args.steps)
         launches = csdr_b200.kernel_launches() - launches0
+        if args.dump_outputs and rank == 0:                      # before the sustained run below overwrites y
+            cols = dump_columns(n_out)
+            dumped = {"fir_bank_out": torch.view_as_real(y[:, torch.from_numpy(cols).to(dev)]).cpu().numpy(), "fir_bank_out_cols": cols.astype(np.float64)}
         sus_ms, sus_n = (per_kernel_ms, args.steps) if args.quick else sustained(fir_step)
+    if args.dump_outputs and rank == 0:
+        dump_outputs(args.dump_outputs, dumped)
     samples_per_step = CHANNELS * N_IN
     value = world * samples_per_step * args.steps / total_ms / 1e3                                   # Msamples/s, whole job
     if args.quick:
@@ -563,7 +588,12 @@ def main():
     ap.add_argument("--no-cpu-baseline", action="store_true")
     ap.add_argument("--no-extra", action="store_true", help="skip the config 3/4/5 legs")
     ap.add_argument("--quick", action="store_true", help="device-resident leg only (for ncu runs): no clock hold loop, no e2e, no CPU baseline")
+    ap.add_argument("--dump-outputs", metavar="DIR", help="write the last timed step's output (sampled, float32) as DIR/<name>.npy")
     args = ap.parse_args()
+    if args.steps < 1:
+        ap.error("--steps must be at least 1")
+    if args.dump_outputs and args.impl != "b200":
+        ap.error("--dump-outputs writes the GPU path's output: it needs --impl b200")
     args.warmup = max(args.warmup, 3) if args.impl == "b200" else max(args.warmup, 1)
     if args.impl == "reference":
         run_reference(args)

@@ -23,5 +23,5 @@ def oracle():
 def ref():
     from oracle.pyoracle import Ref, have_ref
     if not have_ref():
-        pytest.skip("oracle/_ref/libcsdr_ref.so not built (needs /root/reference at build time)")
+        pytest.skip("oracle/_ref/libcsdr_ref.so not built (set CSDR_REFERENCE to the csdr sources at build time)")
     return Ref()

@@ -15,6 +15,7 @@ import pytest
 pytestmark = pytest.mark.gpu
 
 torch = pytest.importorskip("torch")
+REF = np.load(Path(__file__).parent / "golden" / "ref_outputs.npz")         # the compiled reference on the seeded inputs below (make_ref_outputs.py)
 TOL = 1e-5                                                              # BASELINE.json north_star: 1e-5 relative RMS for float blocks
 
 
@@ -33,6 +34,14 @@ def _dev(a):
 
 def _cplx(rng, *shape, amp=1.0):
     return ((rng.uniform(-1, 1, shape) + 1j * rng.uniform(-1, 1, shape)) * amp).astype(np.complex64)
+
+
+def _at(y, key):
+    """(y at the positions where the reference's output is stored, the stored values); the lengths must match"""
+    from oracle.pyoracle import pick_idx
+    n, want = int(REF[key + "_n"]), REF[key]
+    assert y.size == n, (key, y.size, n)
+    return y[pick_idx(n, want.size)], want
 
 
 def _rel(y, ref):
@@ -174,18 +183,18 @@ def test_fastddc_fold_path_ragged_banks(gpu, oracle, channels, nblocks):
 
 
 # ------------------------------------------------------------------------------------------ config 2 vs the compiled reference
-def test_config2_against_compiled_reference_8x262144(gpu, ref):
-    """SURVEY 8(d): config 2 checked against oracle/_ref (the unmodified reference build) on >= 8 channels x the first 262 144 samples."""
+def test_config2_against_compiled_reference_8x262144(gpu):
+    """SURVEY 8(d): config 2 checked against the unmodified reference build on >= 8 channels x the first 262 144 samples
+    (its outputs at 512 seeded positions per channel, tests/golden/ref_outputs.npz)."""
     T, D, C, N = 199, 10, 8, 262_144
     taps = gpu.firdes_lowpass_f(T, 0.5 / D)
     x = np.stack([_cplx(np.random.default_rng(100 + c), N) for c in range(C)])
     y = gpu.fir_decimate_bank_cc(_dev(x), D, taps).cpu().numpy()
-    rtaps = ref.firdes_lowpass_f(T, 0.5 / D)
     worst = 0.0
     for c in range(C):
-        e = _rel(y[c], ref.fir_decimate_cc(x[c], D, rtaps)); worst = max(worst, e)
+        e = _rel(*_at(y[c], f"cfg2_ch{c}")); worst = max(worst, e)
         assert e < TOL, f"channel {c}: rel-RMS {e:.3e} vs the compiled reference (bar {TOL})"
-    print(f"config 2 vs oracle/_ref, 8 ch x 262144: worst rel-RMS {worst:.2e}")
+    print(f"config 2 vs the reference build, 8 ch x 262144: worst rel-RMS {worst:.2e}")
 
 
 def test_config2_full_size_every_32nd_channel(gpu, oracle):

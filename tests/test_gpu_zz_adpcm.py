@@ -8,7 +8,7 @@ import numpy as np
 import pytest
 
 sys.path.insert(0, str(Path(__file__).resolve().parent))
-from test_gpu_cli import clis, run_graph  # noqa: E402,F401
+from test_gpu_cli import arr, clis, run_graph  # noqa: E402,F401
 
 pytestmark = pytest.mark.gpu
 torch = pytest.importorskip("torch")
@@ -63,6 +63,6 @@ def test_openwebrx_waterfall_chain(clis):
     half = np.arange(4096, dtype=np.float32).tobytes()
     assert run_graph(ours, ["fft_exchange_sides_ff 1024"], half) == run_graph(ref, ["fft_exchange_sides_ff 1024"], half)
     stages = ["fft_cc 1024 2048", "logaveragepower_cf -70 1024 4", "fft_exchange_sides_ff 1024", "compress_fft_adpcm_f_u8 1024"]
-    a = np.frombuffer(run_graph(ours, stages, z), np.uint8); b = np.frombuffer(run_graph(ref, stages, z), np.uint8)
+    a = arr(run_graph(ours, stages, z), np.uint8); b = arr(run_graph(ref, stages, z), np.uint8)
     assert a.size == b.size and a.size >= 4 * 517
     assert np.mean(a == b) > 0.95                                          # a centi-dB step that flips perturbs the next few ADPCM nibbles

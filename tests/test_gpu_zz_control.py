@@ -13,12 +13,14 @@ import numpy as np
 import pytest
 
 sys.path.insert(0, str(Path(__file__).resolve().parent))
-from test_gpu_cli import clis, rel, run_graph  # noqa: E402,F401
+from test_gpu_cli import arr, clis, rel, run_graph  # noqa: E402,F401
+from reference_cli import recorded  # noqa: E402
 
 pytestmark = pytest.mark.gpu
 torch = pytest.importorskip("torch")
 
 
+@recorded
 def _with_fd(cli, args_before, args_after, line, data, timeout=120):
     """run `cli <args_before> --fd N <args_after>` with `line` already waiting in the pipe behind descriptor N"""
     r, w = os.pipe()
@@ -31,6 +33,7 @@ def _with_fd(cli, args_before, args_after, line, data, timeout=120):
     return p.stdout
 
 
+@recorded
 def _with_fifo(cli, args_before, args_after, line, data, tmp_path, timeout=120):
     """the same through a named FIFO: the CLI blocks in open() until a writer shows up"""
     path = tmp_path / f"ctl_{abs(hash((cli, tuple(args_before), line))) % 10**8}"
@@ -64,15 +67,16 @@ def test_initial_tuning_through_the_control_channel(clis, tmp_path):
         assert _with_fd(cli, ["shift_unroll_cc"], [], "0.2\n", z) == run_graph(cli, ["shift_unroll_cc 0.2"], z)
         assert _with_fd(cli, ["bandpass_fir_fft_cc"], ["0.05"], "-0.1 0.2\n", z) == run_graph(cli, ["bandpass_fir_fft_cc -0.1 0.2 0.05"], z)
     # and the two programs agree with each other on the controlled runs
-    a = np.frombuffer(_with_fd(ours, ["shift_addition_cc"], [], "0.3\n", z), np.complex64)
-    b = np.frombuffer(_with_fd(ref, ["shift_addition_cc"], [], "0.3\n", z), np.complex64)
+    a = arr(_with_fd(ours, ["shift_addition_cc"], [], "0.3\n", z), np.complex64)
+    b = arr(_with_fd(ref, ["shift_addition_cc"], [], "0.3\n", z), np.complex64)
     assert a.size == b.size and rel(a, b) < 1e-5
     spectra_ours = run_graph(ours, ["fastddc_fwd_cc 8"], z); spectra_ref = run_graph(ref, ["fastddc_fwd_cc 8"], z)
-    a = np.frombuffer(_with_fd(ours, ["fastddc_inv_cc"], ["8"], "-0.21\n", spectra_ours), np.complex64)
-    b = np.frombuffer(_with_fd(ref, ["fastddc_inv_cc"], ["8"], "-0.21\n", spectra_ref), np.complex64)
+    a = arr(_with_fd(ours, ["fastddc_inv_cc"], ["8"], "-0.21\n", spectra_ours), np.complex64)
+    b = arr(_with_fd(ref, ["fastddc_inv_cc"], ["8"], "-0.21\n", spectra_ref), np.complex64)
     assert a.size == b.size and a.size > 0 and rel(a, b) < 1e-5
 
 
+@recorded
 def _retune_run(cli, args_before, args_after, first, second, blocks, out_block_bytes, retune_after, timeout=400):
     """Feed `blocks` one by one; the line `second` is written to the control descriptor while the program waits for block `retune_after`, i.e. after it has
     flushed block retune_after - 1 (a reader thread drains stdout; we wait until those bytes are there).  Both CLIs poll right after writing a block
@@ -121,7 +125,7 @@ def test_midstream_retune_at_a_known_block(clis, oracle):
     blocks = [z[k * B:(k + 1) * B].tobytes() for k in range(nb)]
     outs = {}
     for cli in (ours, ref):
-        outs[cli] = np.frombuffer(_retune_run(cli, ["shift_addition_cc"], [], "0.11\n", "-0.23\n", blocks, B * 8, k0), np.complex64)
+        outs[cli] = arr(_retune_run(cli, ["shift_addition_cc"], [], "0.11\n", "-0.23\n", blocks, B * 8, k0), np.complex64)
         assert outs[cli].size == nb * B
     # the oracle's chain: rate 0.11 for blocks 0..k0, then -0.23, the phase continuing (the CLI re-runs shift_addition_init, not the phase)
     a, ph = oracle.shift_addition_cc(z[:(k0 + 1) * B], 0.11, 0.0, 1024)
@@ -142,9 +146,9 @@ def test_midstream_retune_at_a_known_block(clis, oracle):
     isz = N - T + 1
     zb = z[:8 * isz]
     bl = [zb[k * isz:(k + 1) * isz].tobytes() for k in range(8)]
-    o = [np.frombuffer(_retune_run(cli, ["bandpass_fir_fft_cc"], ["0.05"], "-0.1 0.2\n", "0.05 0.3\n", bl, isz * 8, 4), np.complex64) for cli in (ours, ref)]
+    o = [arr(_retune_run(cli, ["bandpass_fir_fft_cc"], ["0.05"], "-0.1 0.2\n", "0.05 0.3\n", bl, isz * 8, 4), np.complex64) for cli in (ours, ref)]
     assert o[0].size == o[1].size and o[0].size >= 8 * isz
     e = rel(o[0][:8 * isz], o[1][:8 * isz])
     assert e < 1e-5, f"bandpass_fir_fft_cc retuned mid-stream: rel-RMS {e:.3e}"
-    static = np.frombuffer(run_graph(ours, ["bandpass_fir_fft_cc -0.1 0.2 0.05"], zb.tobytes()), np.complex64)
+    static = arr(run_graph(ours, ["bandpass_fir_fft_cc -0.1 0.2 0.05"], zb.tobytes()), np.complex64)
     assert rel(o[0][:4 * isz], static[:4 * isz]) < 1e-6 and rel(o[0][6 * isz:8 * isz], static[6 * isz:8 * isz]) > 0.05      # the retune really happened

@@ -9,7 +9,7 @@ import numpy as np
 import pytest
 
 sys.path.insert(0, str(Path(__file__).resolve().parent))
-from test_gpu_cli import clis, rel, run_graph  # noqa: E402,F401  (the CLI suite's fixture and helpers)
+from test_gpu_cli import arr, clis, rel, run_graph  # noqa: E402,F401  (the CLI suite's fixture and helpers)
 
 pytestmark = pytest.mark.gpu
 torch = pytest.importorskip("torch")
@@ -51,6 +51,6 @@ def test_shift_math_command(clis):
     ours, ref = clis
     z = (np.random.default_rng(3).uniform(-1, 1, 50_000) + 1j * np.random.default_rng(4).uniform(-1, 1, 50_000)).astype(np.complex64).tobytes()
     for rate in (0.2, -0.085, 0.4999):
-        a = np.frombuffer(run_graph(ours, [f"shift_math_cc {rate}"], z), np.complex64)
-        b = np.frombuffer(run_graph(ref, [f"shift_math_cc {rate}"], z), np.complex64)
+        a = arr(run_graph(ours, [f"shift_math_cc {rate}"], z), np.complex64)
+        b = arr(run_graph(ref, [f"shift_math_cc {rate}"], z), np.complex64)
         assert a.size == b.size and a.size > 0 and rel(a, b) < 1e-6, rate

@@ -8,7 +8,7 @@ import numpy as np
 import pytest
 
 sys.path.insert(0, str(Path(__file__).resolve().parent))
-from test_gpu_cli import clis, rel, run_graph  # noqa: E402,F401
+from test_gpu_cli import arr, clis, rel, run_graph  # noqa: E402,F401
 
 pytestmark = pytest.mark.gpu
 torch = pytest.importorskip("torch")
@@ -50,6 +50,6 @@ def test_shift_table_command(clis):
     ours, ref = clis
     z = (np.random.default_rng(3).uniform(-1, 1, 100_000) + 1j * np.random.default_rng(4).uniform(-1, 1, 100_000)).astype(np.complex64).tobytes()
     for args in ("0.2", "-0.085", "0.4999 1024"):
-        a = np.frombuffer(run_graph(ours, [f"shift_table_cc {args}"], z), np.complex64)
-        b = np.frombuffer(run_graph(ref, [f"shift_table_cc {args}"], z), np.complex64)
+        a = arr(run_graph(ours, [f"shift_table_cc {args}"], z), np.complex64)
+        b = arr(run_graph(ref, [f"shift_table_cc {args}"], z), np.complex64)
         assert a.size == b.size and a.size > 0 and rel(a, b) < 1e-6, args

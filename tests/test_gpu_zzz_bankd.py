@@ -4,6 +4,7 @@ the oracle over the whole stream, whatever the daemon's block size."""
 import os
 import socket
 import subprocess
+import sys
 import threading
 from pathlib import Path
 
@@ -48,12 +49,14 @@ def oracle_channel(oracle, wide_c64, rate, taps, tail):
 
 
 def MULTI_DEVICES():
-    """device lists for the daemon's --devices mode: one device always; two when the box has them"""
-    try:
-        import torch
-        return ["0", "0,1"] if torch.cuda.device_count() >= 2 else ["0"]
-    except Exception:
-        return ["0"]
+    """device lists for the daemon's --devices mode: one device always; two when the box has them.  Counted as the daemon counts them: the CUDA
+    runtime (csdrb_device_count) in a process of its own.  torch.cuda.device_count() takes NVML's count when NVML answers; on a machine whose
+    NVML listed GPUs the process could not open, "--devices 0,1" failed with "invalid device ordinal" with one GPU usable."""
+    r = subprocess.run([sys.executable, "-c", "import csdr_b200; print(csdr_b200.lib().csdrb_device_count())"], cwd=ROOT,
+                       stdout=subprocess.PIPE, stderr=subprocess.PIPE, text=True, timeout=120)
+    out = r.stdout.split()
+    assert r.returncode == 0 and out and out[-1].lstrip("-").isdigit(), ("csdrb_device_count", r.returncode, r.stdout, r.stderr[-500:])
+    return ["0", "0,1"] if int(out[-1]) >= 2 else ["0"]
 
 
 def stream_used(oracle, n, block):
